@@ -22,6 +22,11 @@ sharded path and by the CPU oracle on every rank's exported shard (merged on ran
 --impl reference : times the reference's CPU implementation of the same path (the oracle port; faiss itself is
 not vendored in /root/reference), rank 0 only.  `value` = the reference's deployed execution shape (16 pool threads, one
 query per task: conf/index-gflags.conf:5, vector_index.cc:54); the all-host-threads number is reported beside it.
+
+--dump-outputs DIR : writes what the last timed step returned (device-resident and e2e paths) as .npy files, one GPU.
+Database, ids and queries come from fixed seeds, and the centroids from the seeded CPU k-means (the GPU k-means sums
+with float atomics, so its centroids vary from run to run), so two builds run with the same arguments can be compared
+output for output.
 """
 import argparse
 import ctypes
@@ -58,7 +63,33 @@ def parse():
                     "when sharded (one NCCL communicator per batch in flight).  The reference serves searches from a 16-thread pool, "
                     "so concurrent batches are the deployed shape (round-1 sweep: 2 -> 1.39 M, 3 -> 1.44 M, 4 -> 1.47 M, 8 -> 1.49 M QPS)")
     ap.add_argument("--verify", type=int, default=256, help="multi-GPU: queries answered by the sharded path AND by the CPU oracle on every rank's shard")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the results of the last timed step as DIR/<name>.npy: distances (float32) "
+                         "and ids (float64) of the device-resident path and of the host-pointer (e2e) path; a seeded sample of "
+                         "query rows (DIR/query_rows.npy) when all rows exceed 64 MB")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200vs":
+        ap.error("--dump-outputs applies to --impl b200vs")
+    return args
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, nq):
+    """Writes {name: [nq, k] array} as out_dir/<name>.npy, float32 / float64 only, at most DUMP_LIMIT bytes in all."""
+    arrays = {n: a.astype(np.float64) if a.dtype == np.int64 else a for n, a in arrays.items()}
+    row_bytes = sum(a.nbytes // nq for a in arrays.values())
+    os.makedirs(out_dir, exist_ok=True)
+    if row_bytes * nq > DUMP_LIMIT:  # sampled rows + their float64 indices + one 4 KB allowance for the .npy headers
+        rows = np.sort(np.random.default_rng(0).choice(nq, (DUMP_LIMIT - 4096) // (row_bytes + 8), replace=False))
+        arrays = {n: a[rows] for n, a in arrays.items()}
+        arrays["query_rows"] = rows.astype(np.float64)
+    for n, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (n, a.dtype)
+        np.save(os.path.join(out_dir, n + ".npy"), np.ascontiguousarray(a))
 
 
 def measured_peaks():
@@ -207,6 +238,8 @@ def main():
     if args.impl == "reference":
         run_reference(args, rank, world)
         return
+    if args.dump_outputs and world > 1:
+        sys.exit("bench.py: --dump-outputs runs on one GPU (the sharded index trains on the GPUs, not reproducibly)")
 
     import torch
     import b200vs
@@ -231,7 +264,12 @@ def main():
     if world == 1:
         chunks = [(a, x.cpu().numpy()) for a, x in gen_chunks(torch, n, d, 1234 + rank, dev)]
         train = np.concatenate([c for _, c in chunks], 0)[:ntrain] if len(chunks) > 1 else chunks[0][1][:ntrain]
-        ix.train(train)
+        if args.dump_outputs:  # the GPU k-means sums with float atomics; the seeded CPU k-means makes the index reproducible
+            import oracle_lib
+            cent = oracle_lib.load().kmeans(oracle_lib.L2, train, nlist, nthreads=os.cpu_count() or 1)
+            ix.set_trained_state(b200vs.ivf_state_blob(cent, b200vs.L2))
+        else:
+            ix.train(train)
         for a, x in chunks:
             for b in range(0, x.shape[0], 32768):  # kBuildVectorIndexBatchSize, src/common/constant.h:173
                 ix.add(x[b:b + 32768], np.arange(a + b + 1, a + b + 1 + min(32768, x.shape[0] - b), dtype=np.int64))
@@ -310,6 +348,8 @@ def main():
         torch.cuda.profiler.stop()
     ms = e0.elapsed_time(e1)
     gpu_launches = launches[0]
+    last = (args.steps - 1) % L  # lane of the last timed step; later passes overwrite lane 0
+    dumped = {"distances": out_d[last].cpu().numpy(), "ids": out_i[last].cpu().numpy()} if args.dump_outputs else {}
     # the same K steps strictly one after another on one stream (per-batch latency view)
     e0, e1 = timed_device(args.steps, 1)
     barrier()
@@ -351,6 +391,11 @@ def main():
     barrier()
     e2e_s = time.perf_counter() - t0
     clocks = sampler.stop()
+    if args.dump_outputs:
+        last = (args.steps - 1) % L  # caller thread (and buffer) of the last timed step
+        dumped.update(e2e_distances=hd[last].numpy().copy(), e2e_ids=hi[last].numpy().copy())
+        if rank == 0:
+            dump_outputs(args.dump_outputs, dumped, nq)
 
     # max over ranks
     if world > 1:

@@ -17,12 +17,3 @@ def pytest_configure(config):
 def oracle():
     import oracle_lib
     return oracle_lib.load()
-
-
-@pytest.fixture(scope="session")
-def ref_simd():
-    import oracle_lib
-    r = oracle_lib.load_ref()
-    if r is None:
-        pytest.skip("oracle/_ref/libdingo_simd_ref.so not built (needs /root/reference at build time)")
-    return r

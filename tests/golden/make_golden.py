@@ -1,9 +1,10 @@
-"""Regenerates tests/golden/simd_kat.json from the REFERENCE's own kernels (oracle/_ref, built from
-/root/reference/src/simd by oracle/Makefile).  Run in the build container only:
+"""Regenerates tests/golden/simd_kat.json and tests/golden/simd_ref_samples.json from the REFERENCE's own kernels
+(oracle/_ref, built from the reference's src/simd by oracle/Makefile).  Needs oracle/_ref, so it runs only where the
+reference tree is available:
     python tests/golden/make_golden.py
 Inputs are reproducible: (a) the reference's unit-test fixture generator (default-seeded std::mt19937,
 test/unit_test/vector/test_vector_index_flat.cc:491-500) restated by oracle_fixture_mt19937, and
-(b) numpy default_rng(seed).standard_normal.  Outputs are the bit patterns returned by
+(b) numpy default_rng(seed) draws.  Outputs are the bit patterns returned by
 fvec_{L2sqr,inner_product}_avx512 (src/simd/distances_avx512.cc:48-143)."""
 import json
 import os
@@ -47,6 +48,42 @@ def main():
     with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "simd_kat.json"), "w") as f:
         json.dump(out, f, indent=1)
     print("wrote", len(cases), "cases")
+    write_samples(r)
+
+
+def write_samples(r):
+    """simd_ref_samples.json: the reference's answers on the seeded inputs that
+    tests/test_oracle_simd.py::test_bitwise_against_reference_objects and
+    tests/test_oracle_search.py::test_calc_distance_pinned_to_reference_kernels draw."""
+    def both(x, y, d):
+        return (hx(r.ref_fvec_L2sqr_avx512(x.ctypes.data, y.ctypes.data, d)),
+                hx(r.ref_fvec_inner_product_avx512(x.ctypes.data, y.ctypes.data, d)))
+
+    dims, per_dim = list(range(1, 70)) + [127, 128, 129, 767, 768, 769, 1536, 4096], 10
+    rng = np.random.default_rng(0)
+    l2, ip = [], []
+    for d in dims:
+        for _ in range(per_dim):
+            x = rng.standard_normal(d).astype(np.float32)
+            y = (rng.standard_normal(d) * 3).astype(np.float32)
+            a, b = both(x, y, d)
+            l2.append(a)
+            ip.append(b)
+    pairs = {"seed": 0, "dims": dims, "pairs_per_dim": per_dim, "l2": l2, "ip": ip}
+
+    rng = np.random.default_rng(3)
+    left = rng.random((5, 77), dtype=np.float32)
+    right = rng.random((6, 77), dtype=np.float32) * 2 - 0.5
+    grid = [[both(left[i], right[j], 77) for j in range(6)] for i in range(5)]
+    calc = {"seed": 3, "left": [5, 77], "right": [6, 77],
+            "l2": [[c[0] for c in row] for row in grid], "ip": [[c[1] for c in row] for row in grid]}
+
+    out = {"source": "reference src/simd compiled by oracle/Makefile (dingo-store dc8c439c), AVX512 variant",
+           "pairs": pairs, "calc_distance": calc}
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "simd_ref_samples.json"), "w") as f:
+        json.dump(out, f, separators=(",", ":"))
+        f.write("\n")
+    print("wrote", len(l2), "pairs and a 5 x 6 calc_distance grid")
 
 
 if __name__ == "__main__":

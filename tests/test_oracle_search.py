@@ -1,5 +1,8 @@
 """Behavioural checks of the oracle's search restatements (the reference's unit tests assert contracts, not
 numbers: SURVEY.md §4) plus cross-checks against float64 numpy brute force."""
+import json
+import os
+
 import numpy as np
 import pytest
 
@@ -169,19 +172,22 @@ def test_hnsw_recall_and_contract(oracle, metric):
 @pytest.mark.parametrize("algorithm", [1, 2])
 def test_calc_distance_pinned_to_reference_kernels(oracle, algorithm):
     """oracle_calc_distance (vector_index_utils.cc:48-124): every entry is the hooked kernel's value — checked against
-    the reference's own src/simd objects (oracle/_ref) when they are built — and the two normalisers differ."""
-    rng = np.random.default_rng(3)
-    left = rng.random((5, 77), dtype=np.float32)
-    right = rng.random((6, 77), dtype=np.float32) * 2 - 0.5
-    ref = oracle_lib.load_ref()
+    what the reference's own src/simd objects returned on these inputs (tests/golden/simd_ref_samples.json) — and the
+    two normalisers differ."""
+    gold = json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "simd_ref_samples.json")))["calc_distance"]
+    rng = np.random.default_rng(gold["seed"])
+    left = rng.random(tuple(gold["left"]), dtype=np.float32)
+    right = rng.random(tuple(gold["right"]), dtype=np.float32) * 2 - 0.5
+    ref_l2 = np.array([[int(h, 16) for h in row] for row in gold["l2"]], np.uint32).view(np.float32)
+    ref_ip = np.array([[int(h, 16) for h in row] for row in gold["ip"]], np.uint32).view(np.float32)
     d2, lo, ro = oracle.calc_distance(algorithm, oracle_lib.L2, left, right)
     ip, _, _ = oracle.calc_distance(algorithm, oracle_lib.IP, left, right)
     assert np.array_equal(lo, left) and np.array_equal(ro, right)
+    assert d2.shape == ref_l2.shape == ip.shape == ref_ip.shape
     for i in range(5):
         for j in range(6):
-            if ref is not None:
-                assert d2[i, j] == ref.ref_fvec_L2sqr_avx512(left[i].ctypes.data, right[j].ctypes.data, 77)
-                assert ip[i, j] == np.float32(1.0) - np.float32(ref.ref_fvec_inner_product_avx512(left[i].ctypes.data, right[j].ctypes.data, 77))
+            assert d2[i, j] == ref_l2[i, j]
+            assert ip[i, j] == np.float32(1.0) - ref_ip[i, j]
             assert abs(d2[i, j] - float(((left[i].astype(np.float64) - right[j]) ** 2).sum())) < 1e-3
     cs, ln, rn = oracle.calc_distance(algorithm, oracle_lib.COSINE, left, right)
     want_l = oracle.normalize_faiss(left) if algorithm == 1 else oracle.normalize_hnsw(left)

@@ -1,14 +1,15 @@
 """Pins the oracle's distance arithmetic: (1) against the reference's known-answer values (SURVEY.md §0 and
-tests/golden/simd_kat.json, produced by the reference's own src/simd objects), (2) bit-for-bit against
-oracle/_ref when that library is present."""
+tests/golden/simd_kat.json), (2) bit-for-bit against the reference's answers on 770 seeded random pairs
+(tests/golden/simd_ref_samples.json).  Both files hold what the reference's own src/simd objects returned
+(tests/golden/make_golden.py)."""
 import json
 import os
 import struct
 
 import numpy as np
-import pytest
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "simd_kat.json")
+SAMPLES = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "simd_ref_samples.json")
 
 
 def hx(f):
@@ -47,14 +48,18 @@ def test_golden_vectors(oracle):
         assert hx(oracle.ip(a, b)) == c["ip"], c
 
 
-def test_bitwise_against_reference_objects(oracle, ref_simd):
-    rng = np.random.default_rng(0)
-    for d in list(range(1, 70)) + [127, 128, 129, 767, 768, 769, 1536, 4096]:
-        for _ in range(10):
+def test_bitwise_against_reference_objects(oracle):
+    gold = json.load(open(SAMPLES))["pairs"]
+    rng = np.random.default_rng(gold["seed"])
+    i = 0
+    for d in gold["dims"]:
+        for _ in range(gold["pairs_per_dim"]):
             x = rng.standard_normal(d).astype(np.float32)
             y = (rng.standard_normal(d) * 3).astype(np.float32)
-            assert oracle.l2sqr(x, y) == ref_simd.ref_fvec_L2sqr_avx512(x.ctypes.data, y.ctypes.data, d)
-            assert oracle.ip(x, y) == ref_simd.ref_fvec_inner_product_avx512(x.ctypes.data, y.ctypes.data, d)
+            assert hx(oracle.l2sqr(x, y)) == gold["l2"][i], (d, i)
+            assert hx(oracle.ip(x, y)) == gold["ip"][i], (d, i)
+            i += 1
+    assert i == len(gold["l2"]) == len(gold["ip"])
 
 
 def test_normalizers(oracle):
