@@ -58,7 +58,15 @@ SearchCtx make_ctx(IndexBase* ix, const b200vs_search_params* sp, cudaStream_t s
   return sc;
 }
 
-void check_search_args(IndexBase* ix, int64_t nq, const float* xq, const b200vs_search_params* sp) {
+// ExtractVectorValue's value-type check (vector_index_utils.cc:502-530): float rows for float indexes, bytes for binary ones
+void require_float(IndexBase* ix) {
+  if (ix->binary()) fail(B200VS_EVECTOR_INVALID, "float vectors given to a binary index");
+}
+void require_binary(IndexBase* ix) {
+  if (!ix->binary()) fail(B200VS_EVECTOR_INVALID, "binary vectors given to a float index");
+}
+
+void check_search_args(IndexBase* ix, int64_t nq, const void* xq, const b200vs_search_params* sp) {
   if (nq <= 0 || !xq) fail(B200VS_EILLEGAL_PARAMETERS, "vector_with_ids is empty");  // flat.cc:208-210
   if (ix->type == B200VS_HNSW && sp && (sp->efsearch < 0 || sp->efsearch > 1024))
     fail(B200VS_EILLEGAL_PARAMETERS, "efsearch is illegal, " + std::to_string(sp->efsearch) + ", must between 0 and 1024");  // hnsw.cc:332-336
@@ -73,7 +81,12 @@ int b200vs_create(b200vs_type type, b200vs_metric metric, int32_t dim, const b20
     if (!out) fail(B200VS_EILLEGAL_PARAMETERS, "out is null");
     *out = nullptr;
     if (dim <= 0) fail(B200VS_EILLEGAL_PARAMETERS, "dimension must be > 0");
-    if (metric != B200VS_L2 && metric != B200VS_IP && metric != B200VS_COSINE) fail(B200VS_EILLEGAL_PARAMETERS, "unsupported metric type");
+    if (type == B200VS_BINARY_FLAT || type == B200VS_BINARY_IVF_FLAT) {  // vector_index_utils.cc:1085-1099, :1117-1130
+      if (metric != B200VS_HAMMING) fail(B200VS_EILLEGAL_PARAMETERS, "binary indexes need metric HAMMING");
+      if (dim % 8 != 0 || dim > 32768) fail(B200VS_EILLEGAL_PARAMETERS, "binary dimension must be a multiple of 8 and at most 32768");
+    } else if (metric != B200VS_L2 && metric != B200VS_IP && metric != B200VS_COSINE) {
+      fail(B200VS_EILLEGAL_PARAMETERS, "unsupported metric type");
+    }
     b200vs_params p;
     memset(&p, 0, sizeof(p));
     if (params) p = *params;
@@ -86,6 +99,8 @@ int b200vs_create(b200vs_type type, b200vs_metric metric, int32_t dim, const b20
       case B200VS_IVF_FLAT: impl = make_ivf_flat(metric, dim, p); break;
       case B200VS_IVF_PQ: impl = make_ivf_pq(metric, dim, p); break;
       case B200VS_HNSW: impl = make_hnsw(metric, dim, p); break;
+      case B200VS_BINARY_FLAT:
+      case B200VS_BINARY_IVF_FLAT: impl = make_binary(type, dim, p); break;
       default: fail(B200VS_EILLEGAL_PARAMETERS, "unknown index type");
     }
     *out = new b200vs_index{impl};
@@ -102,6 +117,7 @@ void b200vs_destroy(b200vs_index* h) {
 int b200vs_train(b200vs_index* h, int64_t n, const float* x) {
   return guarded([&]() -> int {
     IndexBase* ix = get(h);
+    require_float(ix);
     if (n <= 0 || !x) fail(B200VS_EILLEGAL_PARAMETERS, "data size invalid");  // ivf_flat.cc:646-649
     ix->train(n, x);
     return B200VS_OK;
@@ -126,6 +142,7 @@ int64_t b200vs_get_trained_state(b200vs_index* h, void* blob, size_t cap) {
 int b200vs_add_with_ids(b200vs_index* h, int64_t n, const float* x, const int64_t* ids, int upsert) {
   return guarded([&]() -> int {
     IndexBase* ix = get(h);
+    require_float(ix);
     if (n <= 0 || !x || !ids) fail(B200VS_EILLEGAL_PARAMETERS, "vector_with_ids is empty");  // flat.cc:123-125
     ix->add(n, x, ids, upsert != 0);
     return B200VS_OK;
@@ -173,7 +190,7 @@ int b200vs_remove_ids(b200vs_index* h, int64_t n, const int64_t* ids, int64_t* n
     const int64_t r = ix->remove(n, ids);
     if (n_removed) *n_removed = r < 0 ? 0 : r;
     // IVF types: "remove not found vector id" -> EVECTOR_INVALID (ivf_flat.cc:180-184); untrained -> OK (r == -1)
-    if (r == 0 && (ix->type == B200VS_IVF_FLAT || ix->type == B200VS_IVF_PQ)) fail(B200VS_EVECTOR_INVALID, "remove not found vector id");
+    if (r == 0 && (ix->type == B200VS_IVF_FLAT || ix->type == B200VS_IVF_PQ || ix->type == B200VS_BINARY_IVF_FLAT)) fail(B200VS_EVECTOR_INVALID, "remove not found vector id");
     return B200VS_OK;
   });
 }
@@ -182,6 +199,7 @@ int b200vs_search_device(b200vs_index* h, int64_t nq, const float* xq_dev, int32
                          float* out_dist_dev, int64_t* out_ids_dev, void* stream) {
   return guarded([&]() -> int {
     IndexBase* ix = get(h);
+    require_float(ix);
     check_search_args(ix, nq, xq_dev, sp);
     if (k <= 0) return B200VS_OK;  // "topk <= 0 -> OK", flat.cc:212
     if (!out_ids_dev) fail(B200VS_EILLEGAL_PARAMETERS, "null output");
@@ -342,6 +360,7 @@ int b200vs_search(b200vs_index* h, int64_t nq, const float* xq, int32_t k, const
                   int64_t* out_ids) {
   return guarded([&]() -> int {
     IndexBase* ix = get(h);
+    require_float(ix);
     check_search_args(ix, nq, xq, sp);
     if (k <= 0) return B200VS_OK;
     if (!out_ids || !out_dist) fail(B200VS_EILLEGAL_PARAMETERS, "null output");
@@ -368,6 +387,7 @@ int b200vs_range_search(b200vs_index* h, int64_t nq, const float* xq, float radi
                         const b200vs_search_params* sp, float* out_dist, int64_t* out_ids, int32_t* out_counts) {
   return guarded([&]() -> int {
     IndexBase* ix = get(h);
+    require_float(ix);
     check_search_args(ix, nq, xq, sp);
     if (ix->type == B200VS_HNSW) fail(B200VS_EVECTOR_NOT_SUPPORT, "RangeSearch not support in Hnsw!!!");  // hnsw.cc:487-493
     if (max_results <= 0 || !out_ids || !out_dist || !out_counts) fail(B200VS_EILLEGAL_PARAMETERS, "bad range-search outputs");
@@ -493,6 +513,123 @@ int b200vs_calc_distance(int32_t device, int32_t algorithm, b200vs_metric metric
       throw;
     }
     dl.free(); dr.free(); dn.free(); dout.free();
+    cudaStreamDestroy(s);
+    return B200VS_OK;
+  });
+}
+
+// ---- binary (Hamming) indexes ----
+int b200vs_train_binary(b200vs_index* h, int64_t n, const uint8_t* x) {
+  return guarded([&]() -> int {
+    IndexBase* ix = get(h);
+    require_binary(ix);
+    if (n <= 0 || !x) fail(B200VS_EILLEGAL_PARAMETERS, "data size invalid");
+    ix->train_binary(n, x);
+    return B200VS_OK;
+  });
+}
+
+int b200vs_add_binary_with_ids(b200vs_index* h, int64_t n, const uint8_t* x, const int64_t* ids, int upsert) {
+  return guarded([&]() -> int {
+    IndexBase* ix = get(h);
+    require_binary(ix);
+    if (n <= 0 || !x || !ids) fail(B200VS_EILLEGAL_PARAMETERS, "vector_with_ids is empty");
+    ix->add_binary(n, x, ids, upsert != 0);
+    return B200VS_OK;
+  });
+}
+
+int b200vs_search_binary_device(b200vs_index* h, int64_t nq, const uint8_t* xq_dev, int32_t k, const b200vs_search_params* sp,
+                                float* out_dist_dev, int64_t* out_ids_dev, void* stream) {
+  return guarded([&]() -> int {
+    IndexBase* ix = get(h);
+    require_binary(ix);
+    check_search_args(ix, nq, xq_dev, sp);
+    if (k <= 0) return B200VS_OK;
+    if (!out_ids_dev) fail(B200VS_EILLEGAL_PARAMETERS, "null output");
+    std::shared_lock<std::shared_mutex> rl(ix->rw);
+    ix->set_device();
+    LaneGuard lane(ix, (cudaStream_t)stream);
+    ix->reset_stats();
+    SearchCtx sc = make_ctx(ix, sp, lane.stream);
+    ix->search_binary_dev(nq, xq_dev, k, sc, out_dist_dev, (long long*)out_ids_dev, lane.stream);
+    ix->phases_finish(lane.stream);
+    if (!stream) B200VS_CUDA(cudaStreamSynchronize(lane.stream));
+    return B200VS_OK;
+  });
+}
+
+int b200vs_search_binary(b200vs_index* h, int64_t nq, const uint8_t* xq, int32_t k, const b200vs_search_params* sp, float* out_dist,
+                         int64_t* out_ids) {
+  return guarded([&]() -> int {
+    IndexBase* ix = get(h);
+    require_binary(ix);
+    check_search_args(ix, nq, xq, sp);
+    if (k <= 0) return B200VS_OK;
+    if (!out_ids || !out_dist) fail(B200VS_EILLEGAL_PARAMETERS, "null output");
+    std::shared_lock<std::shared_mutex> rl(ix->rw);
+    ix->set_device();
+    LaneGuard lane(ix, nullptr);
+    cudaStream_t s = lane.stream;
+    ix->reset_stats();
+    const size_t qbytes = (size_t)nq * (ix->dim / 8);
+    uint8_t* dq = ix->scratch.alloc<uint8_t>(qbytes);
+    float* dd = ix->scratch.alloc<float>((size_t)nq * k);
+    long long* di = ix->scratch.alloc<long long>((size_t)nq * k);
+    B200VS_CUDA(cudaMemcpyAsync(dq, xq, qbytes, cudaMemcpyHostToDevice, s));
+    SearchCtx sc = make_ctx(ix, sp, s);
+    ix->search_binary_dev(nq, dq, k, sc, dd, di, s);
+    ix->phases_finish(s);
+    B200VS_CUDA(cudaMemcpyAsync(out_dist, dd, (size_t)nq * k * 4, cudaMemcpyDeviceToHost, s));
+    B200VS_CUDA(cudaMemcpyAsync(out_ids, di, (size_t)nq * k * 8, cudaMemcpyDeviceToHost, s));
+    B200VS_CUDA(cudaStreamSynchronize(s));
+    return B200VS_OK;
+  });
+}
+
+int b200vs_range_search_binary(b200vs_index* h, int64_t nq, const uint8_t* xq, float radius, int32_t max_results,
+                               const b200vs_search_params* sp, float* out_dist, int64_t* out_ids, int32_t* out_counts) {
+  return guarded([&]() -> int {
+    IndexBase* ix = get(h);
+    require_binary(ix);
+    check_search_args(ix, nq, xq, sp);
+    if (max_results <= 0 || !out_ids || !out_dist || !out_counts) fail(B200VS_EILLEGAL_PARAMETERS, "bad range-search outputs");
+    std::shared_lock<std::shared_mutex> rl(ix->rw);
+    ix->set_device();
+    LaneGuard lane(ix, nullptr);
+    cudaStream_t s = lane.stream;
+    const size_t qbytes = (size_t)nq * (ix->dim / 8);
+    uint8_t* dq = ix->scratch.alloc<uint8_t>(qbytes);
+    float* dd = ix->scratch.alloc<float>((size_t)nq * max_results);
+    long long* di = ix->scratch.alloc<long long>((size_t)nq * max_results);
+    int* dc = ix->scratch.alloc<int>((size_t)nq);
+    B200VS_CUDA(cudaMemcpyAsync(dq, xq, qbytes, cudaMemcpyHostToDevice, s));
+    SearchCtx sc = make_ctx(ix, sp, s);
+    ix->range_search_binary_dev(nq, dq, radius, max_results, sc, dd, di, dc, s);
+    B200VS_CUDA(cudaMemcpyAsync(out_dist, dd, (size_t)nq * max_results * 4, cudaMemcpyDeviceToHost, s));
+    B200VS_CUDA(cudaMemcpyAsync(out_ids, di, (size_t)nq * max_results * 8, cudaMemcpyDeviceToHost, s));
+    B200VS_CUDA(cudaMemcpyAsync(out_counts, dc, (size_t)nq * 4, cudaMemcpyDeviceToHost, s));
+    B200VS_CUDA(cudaStreamSynchronize(s));
+    return B200VS_OK;
+  });
+}
+
+// VectorCalcDistance, METRIC_TYPE_HAMMING (vector_index_utils.cc:146-149, :333-356)
+int b200vs_calc_distance_binary(int32_t device, int32_t dim_bits, int64_t nl, const uint8_t* left, int64_t nr, const uint8_t* right,
+                                float* out) {
+  return guarded([&]() -> int {
+    if (dim_bits <= 0 || dim_bits % 8 != 0 || dim_bits > 32768 || nl < 0 || nr < 0) fail(B200VS_EILLEGAL_PARAMETERS, "bad distance-matrix shape");
+    if (nl == 0 || nr == 0) return B200VS_OK;
+    if (!left || !right || !out) fail(B200VS_EILLEGAL_PARAMETERS, "null operand");
+    B200VS_CUDA(cudaSetDevice(device));
+    cudaStream_t s = nullptr;
+    B200VS_CUDA(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+    try {
+      binary_pair_distance(dim_bits, nl, left, nr, right, out, s);
+    } catch (...) {
+      cudaStreamSynchronize(s); cudaStreamDestroy(s);
+      throw;
+    }
     cudaStreamDestroy(s);
     return B200VS_OK;
   });

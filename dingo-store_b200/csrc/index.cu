@@ -123,9 +123,10 @@ void IndexBase::save(const std::string& path) {
   if (st_len > 0) get_state(st.data(), st.size());
   const int nl = export_nlist();
   const int64_t n = type == B200VS_HNSW ? 0 : count();  // the HNSW blob already carries rows + labels
+  const size_t row_bytes = binary() ? (size_t)dim / 8 : (size_t)dim * 4;  // binary rows are dim / 8 bytes (the `codes` export)
   std::vector<int64_t> off(nl + 1, 0), ids((size_t)n);
-  std::vector<float> vec((size_t)n * dim);
-  if (n) export_lists(off.data(), vec.data(), nullptr, ids.data());
+  std::vector<unsigned char> vec((size_t)n * row_bytes);
+  if (n) export_lists(off.data(), binary() ? nullptr : reinterpret_cast<float*>(vec.data()), binary() ? vec.data() : nullptr, ids.data());
   FILE* f = fopen(path.c_str(), "wb");
   if (!f) fail(B200VS_EINTERNAL, "cannot open " + path);
   try {
@@ -136,7 +137,7 @@ void IndexBase::save(const std::string& path) {
     wr(f, st.data(), st.size());
     wr(f, off.data(), off.size() * 8);
     wr(f, ids.data(), ids.size() * 8);
-    wr(f, vec.data(), vec.size() * 4);
+    wr(f, vec.data(), vec.size());
   } catch (...) { fclose(f); throw; }
   fclose(f);
 }
@@ -147,6 +148,7 @@ void IndexBase::load(const std::string& path) {
   try {
     FileHdr h;
     rd(f, &h, sizeof(h));
+    const size_t row_bytes = binary() ? (size_t)dim / 8 : (size_t)dim * 4;
     if (memcmp(h.magic, "B2VSIDX1", 8) != 0 || h.type != (int)type || h.metric != (int)metric || h.dim != dim)
       fail(B200VS_EINTERNAL, "index file does not match this index (type / metric / dimension)");
     if (count() != 0) fail(B200VS_EINTERNAL, "load into a non-empty index");
@@ -155,7 +157,7 @@ void IndexBase::load(const std::string& path) {
       fseek(f, 0, SEEK_END);
       const long fsize = ftell(f);
       fseek(f, here, SEEK_SET);
-      const double need = (double)h.state_len + ((double)h.nlist + 1) * 8 + (double)h.count * (8 + (double)dim * 4);
+      const double need = (double)h.state_len + ((double)h.nlist + 1) * 8 + (double)h.count * (8 + (double)row_bytes);
       if (h.state_len < 0 || h.count < 0 || h.nlist < 0 || h.nlist > (1 << 24) || need > (double)(fsize - here))
         fail(B200VS_EINTERNAL, "corrupt index file (header sizes exceed the file)");
     }
@@ -163,15 +165,17 @@ void IndexBase::load(const std::string& path) {
     rd(f, st.data(), st.size());
     if (h.state_len > 0) set_state(st.data(), st.size());
     std::vector<int64_t> off((size_t)h.nlist + 1), ids((size_t)h.count);
-    std::vector<float> vec((size_t)h.count * dim);
+    std::vector<unsigned char> vec((size_t)h.count * row_bytes);
     rd(f, off.data(), off.size() * 8);
     rd(f, ids.data(), ids.size() * 8);
-    rd(f, vec.data(), vec.size() * 4);
+    rd(f, vec.data(), vec.size());
     loading = true;
     try {
       for (int64_t a = 0; a < h.count; a += 32768) {
         const int64_t m = std::min<int64_t>(32768, h.count - a);
-        add(m, vec.data() + (size_t)a * dim, ids.data() + a, false);
+        const unsigned char* rows = vec.data() + (size_t)a * row_bytes;
+        if (binary()) add_binary(m, rows, ids.data() + a, false);
+        else add(m, reinterpret_cast<const float*>(rows), ids.data() + a, false);
       }
     } catch (...) { loading = false; throw; }
     loading = false;

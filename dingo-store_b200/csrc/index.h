@@ -265,6 +265,25 @@ struct IndexBase {
   }
   virtual int resolve_nprobe_api(const SearchCtx& sc) const { (void)sc; return 1; }
 
+  // ---- binary (Hamming) indexes: rows are dim / 8 bytes.  A float index rejects binary vectors (ExtractVectorValue's
+  // value-type check, vector_index_utils.cc:502-530) ----
+  bool binary() const { return type == B200VS_BINARY_FLAT || type == B200VS_BINARY_IVF_FLAT; }
+  virtual void train_binary(int64_t n, const uint8_t* x) { (void)n; (void)x; fail(B200VS_EVECTOR_INVALID, "binary vectors given to a float index"); }
+  virtual void add_binary(int64_t n, const uint8_t* x, const int64_t* ids, bool upsert) {
+    (void)n; (void)x; (void)ids; (void)upsert;
+    fail(B200VS_EVECTOR_INVALID, "binary vectors given to a float index");
+  }
+  // xq_dev: [nq, dim / 8] device bytes; scratch already reset
+  virtual void search_binary_dev(int64_t nq, const uint8_t* xq_dev, int k, const SearchCtx& sc, float* out_dist, long long* out_ids, cudaStream_t s) {
+    (void)nq; (void)xq_dev; (void)k; (void)sc; (void)out_dist; (void)out_ids; (void)s;
+    fail(B200VS_EVECTOR_INVALID, "binary vectors given to a float index");
+  }
+  virtual void range_search_binary_dev(int64_t nq, const uint8_t* xq_dev, float radius, int max_results, const SearchCtx& sc,
+                                       float* out_dist, long long* out_ids, int* out_counts, cudaStream_t s) {
+    (void)nq; (void)xq_dev; (void)radius; (void)max_results; (void)sc; (void)out_dist; (void)out_ids; (void)out_counts; (void)s;
+    fail(B200VS_EVECTOR_INVALID, "binary vectors given to a float index");
+  }
+
   virtual void reconstruct(int64_t n, const int64_t* ids, float* out, uint8_t* found) {
     (void)n; (void)ids; (void)out; (void)found;
     fail(B200VS_EVECTOR_NOT_SUPPORT, "reconstruct is implemented for HNSW and FLAT");
@@ -327,6 +346,9 @@ IndexBase* make_flat(b200vs_metric m, int d, const b200vs_params& p);
 IndexBase* make_ivf_flat(b200vs_metric m, int d, const b200vs_params& p);
 IndexBase* make_ivf_pq(b200vs_metric m, int d, const b200vs_params& p);
 IndexBase* make_hnsw(b200vs_metric m, int d, const b200vs_params& p);
+IndexBase* make_binary(b200vs_type t, int d, const b200vs_params& p);  // BINARY_FLAT / BINARY_IVF_FLAT (binary.cu)
+// out[i*nr + j] = popcount(a_i ^ b_j) over dim_bits (VectorCalcDistance, METRIC_TYPE_HAMMING); a, b: packed host rows
+void binary_pair_distance(int dim_bits, int64_t nl, const uint8_t* a, int64_t nr, const uint8_t* b, float* out, cudaStream_t s);
 
 // ---- generic exact scan + select driver (scan_kernels.cuh) ----
 struct ScanJob {

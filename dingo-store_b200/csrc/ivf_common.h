@@ -168,6 +168,14 @@ struct IvfLists {
 void launch_kmeans_accumulate(const float* x, const long long* assign, int64_t n, int d, float* sums, int* counts,
                               cudaStream_t s);
 
+// faiss rand_perm (public algorithm): the training subsample and the initial centroids of kmeans_gpu
+inline void kmeans_rand_perm(std::vector<int64_t>& perm, int64_t m, int64_t sd) {
+  perm.resize(m);
+  for (int64_t i = 0; i < m; ++i) perm[i] = i;
+  std::mt19937 mt((unsigned)sd);
+  for (int64_t i = 0; i + 1 < m; ++i) { int64_t i2 = i + (int64_t)(mt() % (unsigned long)(m - i)); std::swap(perm[i], perm[i2]); }
+}
+
 // faiss::Clustering-shaped Lloyd k-means with the assignment step on the GPU (public algorithm; the
 // reference reaches it through index_->train at vector_index_ivf_flat.cc:695 / raw_ivf_pq.cc:485).
 // x_host RAW rows; cosine rows are normalised on the device first.  `assign(xd, m, cd, k, out)` labels m device
@@ -176,12 +184,7 @@ template <class AssignFn, class PrepFn>
 void kmeans_gpu(IndexBase* ix, b200vs_metric metric, int d, int64_t n, const float* x_host, int k, int niter,
                 int max_pts, int64_t seed, std::vector<float>& cent, AssignFn assign, PrepFn prepare_ids) {
   cudaStream_t s = ix->stream;
-  auto rand_perm = [](std::vector<int64_t>& perm, int64_t m, int64_t sd) {
-    perm.resize(m);
-    for (int64_t i = 0; i < m; ++i) perm[i] = i;
-    std::mt19937 mt((unsigned)sd);
-    for (int64_t i = 0; i + 1 < m; ++i) { int64_t i2 = i + (int64_t)(mt() % (unsigned long)(m - i)); std::swap(perm[i], perm[i2]); }
-  };
+  auto rand_perm = kmeans_rand_perm;
   std::vector<float> sub;
   const float* xs = x_host;
   int64_t m = n;

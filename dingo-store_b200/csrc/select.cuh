@@ -26,8 +26,8 @@ struct BlockSelect {
   // smem bytes needed for a pool of `cap` entries (+ header)
   __host__ __device__ static size_t smem_bytes(int cap) { return (size_t)cap * 12 + 32; }
 
-  // carve from a 16-byte aligned shared buffer; all threads call
-  __device__ void init(unsigned char* smem, int cap_, int k_) {
+  // view of a pool laid out at `smem` (no initialisation): lets a block keep several pools without holding their pointers
+  __device__ __forceinline__ void attach(unsigned char* smem, int cap_, int k_) {
     cap = cap_; k = k_;
     kid = reinterpret_cast<long long*>(smem);
     kd = reinterpret_cast<uint32_t*>(smem + (size_t)cap * 8);
@@ -35,6 +35,11 @@ struct BlockSelect {
     thr_id = reinterpret_cast<long long*>(hdr);
     thr_d = reinterpret_cast<uint32_t*>(hdr + 8);
     count = reinterpret_cast<int*>(hdr + 12);
+  }
+
+  // carve from a 16-byte aligned shared buffer; all threads call
+  __device__ void init(unsigned char* smem, int cap_, int k_) {
+    attach(smem, cap_, k_);
     if (threadIdx.x == 0) { *count = 0; *thr_d = KEY_SENTINEL_D; *thr_id = KEY_SENTINEL_ID; }
     __syncthreads();
   }

@@ -36,9 +36,12 @@ enum Errno { OK = 0, EINTERNAL = 10000, EILLEGAL_PARAMTETERS = 10010, EVECTOR_IN
 }  // namespace error
 namespace common {
 enum ValueType { FLOAT = 0, UINT8 = 1 };
-enum MetricType { METRIC_TYPE_NONE = 0, METRIC_TYPE_L2 = 1, METRIC_TYPE_INNER_PRODUCT = 2, METRIC_TYPE_COSINE = 3 };
+enum MetricType { METRIC_TYPE_NONE = 0, METRIC_TYPE_L2 = 1, METRIC_TYPE_INNER_PRODUCT = 2, METRIC_TYPE_COSINE = 3,
+                  METRIC_TYPE_HAMMING = 4 };
+// numeric values are internal to this shim; the real enum lives in proto/common.pb.h
 enum VectorIndexType { VECTOR_INDEX_TYPE_NONE = 0, VECTOR_INDEX_TYPE_FLAT = 1, VECTOR_INDEX_TYPE_IVF_FLAT = 2,
-                       VECTOR_INDEX_TYPE_IVF_PQ = 3, VECTOR_INDEX_TYPE_HNSW = 4 };
+                       VECTOR_INDEX_TYPE_IVF_PQ = 3, VECTOR_INDEX_TYPE_HNSW = 4, VECTOR_INDEX_TYPE_BINARY_FLAT = 6,
+                       VECTOR_INDEX_TYPE_BINARY_IVF_FLAT = 7 };
 
 class Vector {
  public:
@@ -50,10 +53,15 @@ class Vector {
   std::vector<float>* mutable_float_values() { return &float_values_; }
   int float_values_size() const { return (int)float_values_.size(); }
   void add_float_values(float v) { float_values_.push_back(v); }
+  // repeated bytes binary_values: one byte per element for the binary index types (vector_index_utils.cc:590-600)
+  const std::vector<std::string>& binary_values() const { return binary_values_; }
+  int binary_values_size() const { return (int)binary_values_.size(); }
+  void add_binary_values(std::string v) { binary_values_.push_back(std::move(v)); }
  private:
   int32_t dimension_ = 0;
   ValueType value_type_ = FLOAT;
   std::vector<float> float_values_;
+  std::vector<std::string> binary_values_;
 };
 class VectorWithId {
  public:
@@ -76,8 +84,10 @@ class VectorSearchParameter {
   SearchIvfParam* mutable_ivf_pq() { return &ivf_pq_; }
   const SearchHnswParam& hnsw() const { return hnsw_; }
   SearchHnswParam* mutable_hnsw() { return &hnsw_; }
+  const SearchIvfParam& binary_ivf_flat() const { return binary_ivf_flat_; }
+  SearchIvfParam* mutable_binary_ivf_flat() { return &binary_ivf_flat_; }
  private:
-  SearchIvfParam ivf_flat_, ivf_pq_;
+  SearchIvfParam ivf_flat_, ivf_pq_, binary_ivf_flat_;
   SearchHnswParam hnsw_;
 };
 struct CreateFlatParam { int32_t dimension_ = 0; MetricType metric_type_ = METRIC_TYPE_L2;
@@ -99,9 +109,14 @@ class VectorIndexParameter {
   CreateIvfPqParam* mutable_ivf_pq_parameter() { return &ivf_pq_; }
   const CreateHnswParam& hnsw_parameter() const { return hnsw_; }
   CreateHnswParam* mutable_hnsw_parameter() { return &hnsw_; }
+  const CreateFlatParam& binary_flat_parameter() const { return binary_flat_; }  // dimension in bits, metric HAMMING
+  CreateFlatParam* mutable_binary_flat_parameter() { return &binary_flat_; }
+  const CreateIvfFlatParam& binary_ivf_flat_parameter() const { return binary_ivf_flat_; }
+  CreateIvfFlatParam* mutable_binary_ivf_flat_parameter() { return &binary_ivf_flat_; }
  private:
   VectorIndexType type_ = VECTOR_INDEX_TYPE_NONE;
   CreateFlatParam flat_; CreateIvfFlatParam ivf_flat_; CreateIvfPqParam ivf_pq_; CreateHnswParam hnsw_;
+  CreateFlatParam binary_flat_; CreateIvfFlatParam binary_ivf_flat_;
 };
 struct RegionEpoch { int64_t conf_version = 0, version = 0; };
 struct Range { std::string start_key, end_key; };
@@ -200,6 +215,7 @@ class VectorIndex {
   virtual void LockWrite() = 0;
   virtual void UnlockWrite() = 0;
   virtual butil::Status Train(std::vector<float>& train_datas) = 0;
+  virtual butil::Status Train(std::vector<uint8_t>& /*train_datas*/) { return butil::Status::OK(); }  // vector_index.h:195
   virtual butil::Status Train(const std::vector<pb::common::VectorWithId>& vectors) = 0;
   virtual bool NeedToRebuild() = 0;
   virtual bool NeedTrain() { return false; }

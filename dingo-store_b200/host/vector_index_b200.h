@@ -1,8 +1,8 @@
 // vector_index_b200.h — drop-in subclass of dingodb::VectorIndex backed by libb200vs (include/b200vs.h).
 //
-// One class serves the four plugin types; VectorIndexFactory::New{Flat,IvfFlat,IvfPq,Hnsw}
+// One class serves the six plugin types; VectorIndexFactory::New{Flat,IvfFlat,IvfPq,Hnsw,BinaryFlat,BinaryIvfFlat}
 // (src/vector/vector_index_factory.cc:40-95) would return it instead of VectorIndexFlat / VectorIndexIvfFlat /
-// VectorIndexIvfPq / VectorIndexHnsw.  The class does only what the reference plugins do around their faiss /
+// VectorIndexIvfPq / VectorIndexHnsw and their faiss::IndexBinary instantiations.  The class does only what the reference plugins do around their faiss /
 // hnswlib calls: argument checks with the same status codes, pb -> flat-array marshalling
 // (CheckVectorDimension / ExtractVectorValue / FillSearchResult, src/vector/vector_index_utils.cc:502-655), filter
 // lowering, and the write lock bookkeeping; all arithmetic is behind the C ABI.
@@ -55,6 +55,7 @@ class VectorIndexB200 : public VectorIndex {
   void UnlockWrite() override { write_gate_.unlock(); }
   butil::Status Train(std::vector<float>& train_datas) override;
   butil::Status Train(const std::vector<pb::common::VectorWithId>& vectors) override;
+  butil::Status Train(std::vector<uint8_t>& train_datas) override;  // binary types: dim / 8 bytes per row
   bool NeedToRebuild() override { return false; }
   bool NeedTrain() override;
   bool IsTrained() override;
@@ -70,21 +71,30 @@ class VectorIndexB200 : public VectorIndex {
  private:
   butil::Status AddOrUpsert(const std::vector<pb::common::VectorWithId>& vector_with_ids, bool is_upsert);
   butil::Status ToStatus(int rc) const;
+  int32_t SearchNprobe(const pb::common::VectorSearchParameter& parameter) const;
 
   b200vs_index* index_ = nullptr;
-  int32_t dimension_ = 0;
+  int32_t dimension_ = 0;  // bits for the binary types
+  bool binary_ = false;     // BINARY_FLAT / BINARY_IVF_FLAT: rows are UINT8 binary_values
   pb::common::MetricType metric_type_ = pb::common::METRIC_TYPE_NONE;
   std::shared_mutex write_gate_;  // LockWrite/UnlockWrite of the snapshot path; reads and writes lock inside the library
 };
 
 // VectorIndexUtils::CalcDistanceEntry (src/vector/vector_index_utils.cc:48-76) over the C ABI: same operand meaning
 // (algorithm_type = pb::index::AlgorithmType: 1 FAISS, 2 HNSWLIB; metric; is_return_normlize) and the same error codes.
+// METRIC_TYPE_HAMMING reads the operands' binary_values (utils.cc:146-149, :333-356).
 class VectorIndexB200Utils {
  public:
   static butil::Status CalcDistance(int algorithm_type, pb::common::MetricType metric_type, const std::vector<pb::common::Vector>& op_left_vectors,
                                     const std::vector<pb::common::Vector>& op_right_vectors, bool is_return_normlize,
                                     std::vector<std::vector<float>>& distances, std::vector<pb::common::Vector>& result_op_left_vectors,
                                     std::vector<pb::common::Vector>& result_op_right_vectors, int device = 0);
+
+ private:
+  static butil::Status CalcHammingDistance(int algorithm_type, const std::vector<pb::common::Vector>& op_left_vectors,
+                                           const std::vector<pb::common::Vector>& op_right_vectors, bool is_return_normlize,
+                                           std::vector<std::vector<float>>& distances, std::vector<pb::common::Vector>& result_op_left_vectors,
+                                           std::vector<pb::common::Vector>& result_op_right_vectors, int device);
 };
 
 // The inner loop of VectorReader::BruteForceSearch (src/vector/vector_reader.cc:1873-2048): the caller keeps the RocksDB

@@ -13,8 +13,9 @@ PKG_ROOT = os.path.abspath(os.path.join(_HERE, "..", ".."))       # dingo-store_
 REPO_ROOT = os.path.abspath(os.path.join(PKG_ROOT, ".."))
 LIB_PATH = os.path.join(PKG_ROOT, "libb200vs.so")
 
-FLAT, IVF_FLAT, IVF_PQ, HNSW = 0, 1, 2, 3
-L2, IP, COSINE = 1, 2, 3
+FLAT, IVF_FLAT, IVF_PQ, HNSW, BINARY_FLAT, BINARY_IVF_FLAT = 0, 1, 2, 3, 4, 5
+L2, IP, COSINE, HAMMING = 1, 2, 3, 4
+BINARY_TYPES = (BINARY_FLAT, BINARY_IVF_FLAT)
 OK, EILLEGAL_PARAMETERS, EVECTOR_INVALID, EVECTOR_NOT_TRAIN, EVECTOR_NOT_SUPPORT, EINTERNAL, EVECTOR_ID_DUPLICATED = range(7)
 
 # every symbol include/b200vs.h declares (checked by tests/test_abi.py without a GPU)
@@ -29,6 +30,8 @@ ABI_SYMBOLS = [
     "b200vs_shard_unique_id", "b200vs_shard_create", "b200vs_shard_destroy", "b200vs_shard_list_range", "b200vs_shard_train",
     "b200vs_shard_broadcast_state", "b200vs_shard_add", "b200vs_shard_add_device", "b200vs_shard_remove_ids", "b200vs_shard_plan_add_device",
     "b200vs_shard_plan_commit", "b200vs_shard_search", "b200vs_shard_search_device",
+    "b200vs_train_binary", "b200vs_add_binary_with_ids", "b200vs_search_binary", "b200vs_search_binary_device",
+    "b200vs_range_search_binary", "b200vs_calc_distance_binary",
 ]
 
 
@@ -120,6 +123,12 @@ def lib():
     L.b200vs_shard_plan_commit.argtypes = [vp]
     L.b200vs_shard_search.argtypes = [vp, i64, i64, vp, i32, ctypes.POINTER(SearchParams), vp, vp]
     L.b200vs_shard_search_device.argtypes = [vp, i64, i64, vp, i32, ctypes.POINTER(SearchParams), vp, vp, vp]
+    L.b200vs_train_binary.argtypes = [vp, i64, vp]
+    L.b200vs_add_binary_with_ids.argtypes = [vp, i64, vp, vp, ctypes.c_int]
+    L.b200vs_search_binary.argtypes = [vp, i64, vp, i32, ctypes.POINTER(SearchParams), vp, vp]
+    L.b200vs_search_binary_device.argtypes = [vp, i64, vp, i32, ctypes.POINTER(SearchParams), vp, vp, vp]
+    L.b200vs_range_search_binary.argtypes = [vp, i64, vp, f32, i32, ctypes.POINTER(SearchParams), vp, vp, vp]
+    L.b200vs_calc_distance_binary.argtypes = [i32, i32, i64, vp, i64, vp, vp]
     _lib = L
     return L
 
@@ -136,6 +145,10 @@ def _f32(a):
 
 def _i64(a):
     return np.ascontiguousarray(a, dtype=np.int64)
+
+
+def _u8(a):
+    return np.ascontiguousarray(a, dtype=np.uint8)
 
 
 def make_search_params(nprobe=0, efsearch=0, id_range=None, sorted_ids=None, negate=False, exact_only=False):
@@ -177,8 +190,25 @@ class Index:
         except Exception:
             pass
 
+    @property
+    def binary(self):
+        """BINARY_FLAT / BINARY_IVF_FLAT: dim is in bits, rows are uint8 [n, dim // 8]."""
+        return self.type in BINARY_TYPES
+
+    def _rows(self, x):
+        """(contiguous rows, row count) in the index's value type."""
+        if self.binary:
+            x = _u8(x)
+            return x, (x.shape[0] if x.ndim == 2 else x.size // (self.dim // 8))
+        x = _f32(x)
+        return x, (x.shape[0] if x.ndim == 2 else x.size // self.dim)
+
     # ---- write path ----
     def train(self, x):
+        if self.binary:
+            x, n = self._rows(x)
+            _check(self.L.b200vs_train_binary(self.h, n, x.ctypes.data if x.size else None))
+            return
         x = _f32(x)
         n = x.shape[0] if x.ndim == 2 else x.size // self.dim
         _check(self.L.b200vs_train(self.h, n, x.ctypes.data))
@@ -198,6 +228,10 @@ class Index:
         return buf[:got]
 
     def add(self, x, ids, upsert=False):
+        if self.binary:
+            x, ids = _u8(x), _i64(ids)
+            _check(self.L.b200vs_add_binary_with_ids(self.h, ids.size, x.ctypes.data if x.size else None, ids.ctypes.data if ids.size else None, int(upsert)))
+            return
         x, ids = _f32(x), _i64(ids)
         _check(self.L.b200vs_add_with_ids(self.h, ids.size, x.ctypes.data if x.size else None, ids.ctypes.data if ids.size else None, int(upsert)))
 
@@ -222,12 +256,12 @@ class Index:
 
     # ---- read path ----
     def search(self, xq, k, **kw):
-        xq = _f32(xq)
-        nq = xq.shape[0] if xq.ndim == 2 else xq.size // self.dim
+        xq, nq = self._rows(xq)
         sp, keep = make_search_params(**kw)
         D = np.zeros((nq, max(k, 0)), dtype=np.float32)
         I = np.full((nq, max(k, 0)), -1, dtype=np.int64)
-        _check(self.L.b200vs_search(self.h, nq, xq.ctypes.data if xq.size else None, k, ctypes.byref(sp), D.ctypes.data, I.ctypes.data))
+        fn = self.L.b200vs_search_binary if self.binary else self.L.b200vs_search
+        _check(fn(self.h, nq, xq.ctypes.data if xq.size else None, k, ctypes.byref(sp), D.ctypes.data, I.ctypes.data))
         return D, I
 
     def search_raw(self, nq, xq_ptr, k, out_dist_ptr, out_ids_ptr, sp=None):
@@ -235,7 +269,8 @@ class Index:
         _check(self.L.b200vs_search(self.h, nq, xq_ptr, k, ctypes.byref(sp) if sp is not None else None, out_dist_ptr, out_ids_ptr))
 
     def search_device(self, nq, xq_dev_ptr, k, out_dist_dev_ptr, out_ids_dev_ptr, stream=None, sp=None):
-        _check(self.L.b200vs_search_device(self.h, nq, xq_dev_ptr, k, ctypes.byref(sp) if sp is not None else None,
+        fn = self.L.b200vs_search_binary_device if self.binary else self.L.b200vs_search_device
+        _check(fn(self.h, nq, xq_dev_ptr, k, ctypes.byref(sp) if sp is not None else None,
                                            out_dist_dev_ptr, out_ids_dev_ptr, stream))
 
     def coarse_device(self, nq, xq_dev_ptr, nprobe, list_begin, list_end, out_score_dev_ptr, out_lists_dev_ptr, stream=None):
@@ -246,13 +281,13 @@ class Index:
                                                   out_dist_dev_ptr, out_ids_dev_ptr, stream))
 
     def range_search(self, xq, radius, max_results=1024, **kw):
-        xq = _f32(xq)
-        nq = xq.shape[0] if xq.ndim == 2 else xq.size // self.dim
+        xq, nq = self._rows(xq)
         sp, keep = make_search_params(**kw)
         D = np.zeros((nq, max_results), dtype=np.float32)
         I = np.full((nq, max_results), -1, dtype=np.int64)
         C = np.zeros(nq, dtype=np.int32)
-        _check(self.L.b200vs_range_search(self.h, nq, xq.ctypes.data if xq.size else None, float(radius), max_results,
+        fn = self.L.b200vs_range_search_binary if self.binary else self.L.b200vs_range_search
+        _check(fn(self.h, nq, xq.ctypes.data if xq.size else None, float(radius), max_results,
                                           ctypes.byref(sp), D.ctypes.data, I.ctypes.data, C.ctypes.data))
         return D, I, C
 
@@ -292,6 +327,9 @@ class Index:
         _check(self.L.b200vs_set_profiling(self.h, int(bool(on))))
 
     def export_lists(self, nlist, with_vectors=True, code_size=0):
+        """(list_off, vectors, codes, ids).  Binary indexes return their rows as codes [n, dim // 8] (vectors None)."""
+        if self.binary:
+            with_vectors, code_size = False, self.dim // 8
         n = self.get_count()
         off = np.zeros(nlist + 1, dtype=np.int64)
         vec = np.zeros((n, self.dim), dtype=np.float32) if with_vectors else None
@@ -418,6 +456,13 @@ def ivf_state_blob(centroids, metric):
     return np.concatenate([hdr.view(np.uint8), c.reshape(-1).view(np.uint8)])
 
 
+def binary_ivf_state_blob(centroids):
+    """Trained-state blob of a BINARY_IVF_FLAT index: packed centroids uint8 [nlist, dim // 8] (DESIGN.md §5)."""
+    c = _u8(centroids)
+    hdr = np.array([0x46564942, c.shape[0], c.shape[1] * 8, HAMMING], dtype=np.int64)
+    return np.concatenate([hdr.view(np.uint8), c.reshape(-1)])
+
+
 def merge_topk_device(device, nparts, nq, k, parts_dist_ptr, parts_ids_ptr, out_dist_ptr, out_ids_ptr, stream=None):
     _check(lib().b200vs_merge_topk_device(device, nparts, nq, k, parts_dist_ptr, parts_ids_ptr, out_dist_ptr, out_ids_ptr, stream))
 
@@ -437,6 +482,16 @@ def calc_distance(algorithm, metric, left, right, return_normalized=False, devic
                                       right.ctypes.data if right.size else None, out.ctypes.data if out.size else None,
                                       lo.ctypes.data if lo is not None and lo.size else None, ro.ctypes.data if ro is not None and ro.size else None))
     return (out, lo, ro) if return_normalized else out
+
+
+def calc_distance_binary(left, right, device=0):
+    """Pairwise Hamming matrix [nl, nr] of packed rows uint8 [n, dim // 8] (VectorCalcDistance, METRIC_TYPE_HAMMING)."""
+    left, right = _u8(left), _u8(right)
+    nl, nr = left.shape[0], right.shape[0]
+    out = np.zeros((nl, nr), dtype=np.float32)
+    _check(lib().b200vs_calc_distance_binary(device, left.shape[1] * 8, nl, left.ctypes.data if left.size else None, nr,
+                                             right.ctypes.data if right.size else None, out.ctypes.data if out.size else None))
+    return out
 
 
 class BruteForceScan:
